@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- the hot-path benchmark (driver contract).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|c3|c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|c3|c4|c5] [--dump-outputs DIR]
 
 One "step" = one pass of the workload's op list over one batch of synthetic frames.  Default workload = BASELINE.json
 configs[1] ("c2"): the filter2D / sepFilter2D / GaussianBlur sweep 3x3..31x31 on 3840x2160 CV_8UC1 and CV_32FC1.
@@ -11,6 +11,8 @@ kernel with the largest share of the step, `per_op` for every op, `cpu_baseline`
 (oracle/_ref, or the C port when that is absent) on a bounded sample, `clocks` sampled during the timed region.
 Multi-GPU (torchrun): frames shard across ranks (weak scaling); the only collective is an NCCL broadcast of the filter
 taps / template per step.
+--dump-outputs DIR: after the timed steps, rank 0 writes what every op of the workload returned in the last timed step as
+DIR/<op>.npy (see dump_outputs); the inputs are seeded, so two builds run with the same arguments can be compared output by output.
 """
 import argparse
 import json
@@ -255,7 +257,45 @@ def make_extra(ops, rng, need_device):
     return extra
 
 
-def measure_device(workload, steps, W, use_graph, rank, world, local, rng, sample_clocks=True):
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(ops, out_dir, dev):
+    """What each op returned in the last step, as DIR/<op name>[_<i>].npy (one file per array of the result, in the order the op returns
+    them): float64 results stay float64, 8- and 16-bit results and float32 become float32, wider integers float64 -- all exact.  The files
+    hold at most DUMP_BYTES together: an array larger than its share is written as a fixed sample of its elements (flattened, at sorted
+    positions drawn from a generator seeded with the file name), the same positions in every run."""
+    import zlib
+    import torch
+    arrays = []
+
+    def leaves(name, x):
+        if isinstance(x, (list, tuple)):
+            items = [v for v in x if v is not None]
+            for i, v in enumerate(items):
+                leaves(name if len(items) == 1 else "%s_%d" % (name, i), v)
+        elif x is not None:
+            arrays.append((name, x))
+    for op in ops:
+        leaves(op["name"], op["_out"])
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // max(1, len(arrays)) - 256          # 256: room for the .npy header
+    for name, a in arrays:
+        dt = np.float64 if str(a.dtype).endswith(("float64", "int32", "int64")) else np.float32
+        n = int(a.numel()) if isinstance(a, torch.Tensor) else int(a.size)
+        keep = share // np.dtype(dt).itemsize
+        idx = None
+        if n > keep:
+            idx = np.sort(np.random.default_rng(zlib.crc32(name.encode())).integers(0, n, keep))
+        if isinstance(a, torch.Tensor):
+            t = a.reshape(-1)[torch.from_numpy(idx).to(dev)] if idx is not None else a
+            v = t.cpu().numpy()
+        else:
+            v = np.asarray(a).reshape(-1)[idx] if idx is not None else np.asarray(a)
+        np.save(os.path.join(out_dir, name + ".npy"), v.astype(dt))
+
+
+def measure_device(workload, steps, W, use_graph, rank, world, local, rng, sample_clocks=True, dump_dir=None):
     """device-resident pass of one workload: returns (result dict, ops, extra, bufs).  value = Mpix/s over `steps` steps (CUDA events, max over ranks)"""
     import torch
     import torch.distributed as dist
@@ -267,8 +307,8 @@ def measure_device(workload, steps, W, use_graph, rank, world, local, rng, sampl
     # device-resident inputs / outputs: one buffer per distinct spec (every op's in+out working set > L2)
     bufs = {}
 
-    def buf(spec, fill):
-        key = (spec[0], np.dtype(spec[1]).str, fill)
+    def buf(spec, fill, owner=None):
+        key = (spec[0], np.dtype(spec[1]).str, fill, owner)
         if key not in bufs:
             shp, dt = spec
             tdt = torch.uint8 if np.dtype(dt) == np.uint8 else torch.float32
@@ -282,7 +322,9 @@ def measure_device(workload, steps, W, use_graph, rank, world, local, rng, sampl
 
     for op in ops:
         op["_src"] = buf(op["src"], True)
-        op["_dst"] = buf(op["dst"], False) if op["dst"] is not None else None
+        # ops of one shape share a destination, so a step leaves only the last one's result in it; to dump every op's result, each op
+        # gets its own (before the graph is captured)
+        op["_dst"] = buf(op["dst"], False, op["name"] if dump_dir else None) if op["dst"] is not None else None
     if workload == "c4":
         extra["templ"] = ops[0]["_src"][0, 700:764, 1000:1064, 0].contiguous()
 
@@ -330,7 +372,7 @@ def measure_device(workload, steps, W, use_graph, rank, world, local, rng, sampl
         for i, op in enumerate(ops):
             if record:
                 ev[i][0].record()
-            run_op(cvb, op, op["_src"], op["_dst"], extra)
+            op["_out"] = run_op(cvb, op, op["_src"], op["_dst"], extra)    # in a captured graph: its static outputs, rewritten by every replay
             if record:
                 ev[i][1].record()
 
@@ -391,6 +433,8 @@ def measure_device(workload, steps, W, use_graph, rank, world, local, rng, sampl
     e1.record()
     barrier()
     total_ms = e0.elapsed_time(e1)
+    if dump_dir and rank == 0:
+        dump_outputs(ops, dump_dir, dev)
     sampler.stop_flag = True
     if sample_clocks:
         sampler.join(timeout=2)
@@ -485,7 +529,7 @@ def measure_e2e(workload, ops, extra, bufs, steps, rank, world, local):
         if key not in hb:
             a = drv.pinned_frames(spec[0], spec[1])
             if fill:
-                t = bufs[(spec[0], np.dtype(spec[1]).str, True)] if src_t is None else src_t
+                t = bufs[(spec[0], np.dtype(spec[1]).str, True, None)] if src_t is None else src_t
                 a[...] = t.cpu().numpy()
             hb[key] = a
         return hb[key]
@@ -576,6 +620,8 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="issue every launch from the host each step instead of replaying a captured CUDA graph")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the short C3/C4/C5 passes that ride along with the default (C2) workload")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what each op of the workload returned in the last one "
+                                                          "as DIR/<op>.npy (float32 / float64, at most 64 MB in all)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     rng = np.random.default_rng(0x5EED0000 + 2 + rank)
@@ -619,7 +665,7 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     dev = torch.device("cuda", local)
-    res, ops, extra, bufs = measure_device(args.workload, args.steps, W, not args.no_graph, rank, world, local, rng)
+    res, ops, extra, bufs = measure_device(args.workload, args.steps, W, not args.no_graph, rank, world, local, rng, dump_dir=args.dump_outputs)
     value, total_ms, per_op, roofline, launches = res["value"], res["total_ms"], res["per_op"], res["roofline"], res["launches"]
     graph_note, host_enqueue_ms, desc = res["graph_note"], res["host_enqueue_ms"], res["desc"]
 

@@ -62,8 +62,11 @@ def build(jobs=None, force=False, verbose=False):
                 failed = True
     if failed:
         raise RuntimeError("b200cv: compilation failed")
-    if force or not os.path.exists(LIB) or any(os.path.getmtime(o) > os.path.getmtime(LIB) for o in objs):
-        cmd = [NVCC, "-shared", "-o", LIB] + objs + ["-cudart", "static", "-Xlinker", "--no-undefined", "-lpthread", "-ldl", "-lrt"]
+    if force or not os.path.exists(LIB) or any(os.path.getmtime(o) > os.path.getmtime(LIB) for o in objs + [os.path.abspath(__file__)]):
+        # the soname lets a library that needs libb200cv.so (the reference built with the HAL header) use the copy already loaded,
+        # wherever that library was built or moved
+        cmd = [NVCC, "-shared", "-o", LIB] + objs + ["-cudart", "static", "-Xlinker", "--no-undefined", "-Xlinker", "-soname=libb200cv.so",
+                                                     "-lpthread", "-ldl", "-lrt"]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode != 0:
             sys.stderr.write(r.stdout + r.stderr)

@@ -15,6 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 REF_LIB = os.path.join(HERE, "_ref", "libocvref.so")
 REF_HAL_LIB = os.path.join(HERE, "_ref", "libocvref_hal.so")   # the reference with hal/b200cv_hal_replacement.hpp registered (integration proof)
 PORT_LIB = os.path.join(HERE, "_build", "liboracle_port.so")
+B200_LIB = os.path.join(os.path.dirname(HERE), "opencv_b200", "lib", "libb200cv.so")
 
 CV_8U, CV_16S, CV_32F = 0, 3, 5
 _DEPTH = {np.dtype(np.uint8): CV_8U, np.dtype(np.uint16): 2, np.dtype(np.int16): CV_16S, np.dtype(np.float32): CV_32F}
@@ -65,6 +66,10 @@ class Oracle:
         path = _path(kind)
         if not os.path.exists(path):
             raise FileNotFoundError("%s oracle not built: %s" % (kind, path))
+        if kind == "ref_hal":
+            # its libb200cv.so dependency resolves (by soname) to this tree's library loaded first, not to wherever the run path of the
+            # reference build points
+            ctypes.CDLL(B200_LIB)
         self.lib = ctypes.CDLL(path)
         self.pfx = "ref_" if kind in ("ref", "ref_hal") else "port_"
 

@@ -214,7 +214,9 @@ def main():
             hal_objs.append(hobj)
         hlib = os.path.join(OUT, "libocvref_hal.so")
         b200 = os.path.join(repo, "opencv_b200", "lib")
-        ninja.insert(2, "rule linkhal\n  command = g++ -shared -o $out $in -pthread -ldl -lm -Wl,--gc-sections -L%s -lb200cv -Wl,-rpath,%s -Wl,-rpath,$$ORIGIN/../../opencv_b200/lib\n  description = LINK $out\n" % (b200, b200))
+        # ninja hands the command to /bin/sh: the quotes keep $ORIGIN literal, so the library finds libb200cv.so relative to itself
+        # wherever the tree is moved to
+        ninja.insert(2, "rule linkhal\n  command = g++ -shared -o $out $in -pthread -ldl -lm -Wl,--gc-sections -L%s -lb200cv '-Wl,-rpath,$$ORIGIN/../../opencv_b200/lib'\n  description = LINK $out\n" % b200)
         ninja.append("build %s: linkhal %s\n" % (hlib, " ".join(hal_objs)))
         defaults.append(hlib)
     ninja.append("default %s\n" % " ".join(defaults))

@@ -9,8 +9,26 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 
+def pytest_addoption(parser):
+    parser.addoption("--record-reference", action="store_true",
+                     help="record what the reference returns to every test using the `ref` fixture into tests/golden/reference_calls.npz "
+                          "(needs oracle/_ref/libocvref.so; run it over the CPU tests)")
+
+
 def pytest_configure(config):
-    config.addinivalue_line("markers", "gpu: needs a real B200 (run with -m gpu on the GPU box)")
+    config.addinivalue_line("markers", "gpu: needs a real B200 (run with -m gpu on a machine with one)")
+    config.addinivalue_line("markers", "reference_library: checks the reference library itself against constants kept in the repository; "
+                                       "there is nothing to record or replay, it runs only where oracle/_ref is built")
+
+
+_RECORDED = {}
+_REF = []
+
+
+def pytest_sessionfinish(session):
+    if _RECORDED:
+        import reference_replay
+        reference_replay.save(_RECORDED)
 
 
 def _port():
@@ -26,13 +44,23 @@ def port():
     return _port()
 
 
-@pytest.fixture(scope="session")
-def ref():
-    """the unmodified reference built by oracle/build_ref.py (skips when oracle/_ref is absent)"""
+@pytest.fixture()
+def ref(request):
+    """the unmodified reference built by oracle/build_ref.py; where oracle/_ref is absent, its recorded answers to this test
+    (tests/reference_replay.py), and a skip when the test has none"""
     from oracle.api import Oracle, available
-    if not available("ref"):
-        pytest.skip("oracle/_ref/libocvref.so not built")
-    return Oracle("ref")
+    import reference_replay
+    test_id = "%s::%s" % (os.path.basename(str(request.node.fspath)), request.node.name)
+    if available("ref"):
+        if not _REF:
+            _REF.append(Oracle("ref"))
+        if request.config.getoption("--record-reference") and not request.node.get_closest_marker("reference_library"):
+            return reference_replay.Recorder(_REF[0], _port(), _RECORDED, test_id)
+        return _REF[0]
+    archive = reference_replay.recording()
+    if test_id not in archive["tests"]:
+        pytest.skip("oracle/_ref/libocvref.so not built and no recording of this test")
+    return reference_replay.Replay(archive, archive["tests"][test_id], _port(), test_id)
 
 
 @pytest.fixture(scope="session")

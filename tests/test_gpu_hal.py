@@ -178,16 +178,20 @@ def test_cpp_host_mirror(cvb):
 
 
 def test_cv_typed_surface_against_real_opencv_headers(cvb):
-    """tests/cpp/test_cv_surface: opencv_b200/host/b200cv_opencv.hpp compiled with -DB200CV_WITH_OPENCV against the reference's own headers and
-    linked with the reference's core + imgproc (built here by tests/cpp/build_cv_surface.py): cv::InputArray kinds MAT / CUDA_GPU_MAT /
+    """oracle/_ref/test_cv_surface: opencv_b200/host/b200cv_opencv.hpp compiled with -DB200CV_WITH_OPENCV against the reference's own headers and
+    linked with the reference's core + imgproc (built by tests/cpp/build_cv_surface.py): cv::InputArray kinds MAT / CUDA_GPU_MAT /
     CUDA_HOST_MEM, createGaussianFilter(...)->apply(src, dst, stream) as in gpu-basics-similarity.cpp:392-404, each result checked against
     the cv:: call on the CPU inside the binary"""
     import os
     import subprocess
-    exe = os.path.join(os.path.dirname(__file__), "cpp", "test_cv_surface")
+    exe = os.path.join(os.path.dirname(__file__), "..", "oracle", "_ref", "test_cv_surface")
     if not os.path.exists(exe):
-        pytest.skip("tests/cpp/test_cv_surface not built (needs /root/reference at build time)")
-    r = subprocess.run([exe], capture_output=True, text=True, timeout=300)
+        pytest.skip("oracle/_ref/test_cv_surface not built (needs the reference's sources at build time)")
+    # this tree's libraries, whatever run path the binary was linked with where oracle/_ref was built
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    env = dict(os.environ, LD_LIBRARY_PATH=os.pathsep.join([os.path.join(root, "opencv_b200", "lib"), os.path.join(root, "oracle", "_ref")] +
+                                                           [p for p in [os.environ.get("LD_LIBRARY_PATH")] if p]))
+    r = subprocess.run([exe], capture_output=True, text=True, timeout=300, env=env)
     assert r.returncode == 0, r.stdout + r.stderr
     assert "cv surface ok" in r.stdout
 

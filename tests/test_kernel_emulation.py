@@ -11,7 +11,9 @@ import zlib
 import numpy as np
 import pytest
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+from reference_replay import with_twin
+
+ROOT =os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CSRC = os.path.join(ROOT, "opencv_b200", "csrc")
 OUT = os.path.join(ROOT, "tests", "emu", "_build")
 GOLD = os.path.join(ROOT, "tests", "golden")
@@ -343,12 +345,9 @@ def depth_emu():
     return run
 
 
-def test_emulated_depth_cvtcolor_vs_reference(depth_emu, rng):
+def test_emulated_depth_cvtcolor_vs_reference(depth_emu, ref, rng):
     """the kernel source of cvtcolor_depth.cu compiled for the host == the compiled reference, bit for bit (vector bodies and scalar tails)"""
-    from oracle.api import Oracle, available
-    if not available("ref"):
-        pytest.skip("oracle/_ref/libocvref.so not built")
-    ref = Oracle("ref")
+    ref = with_twin(ref, cvtColor=depth_emu)
     for (h, w) in [(9, 29), (5, 64), (3, 7)]:
         f3 = (rng.random((h, w, 3), dtype=np.float32) * 1.5 - 0.25).astype(np.float32)
         w3 = rng.integers(0, 65536, (h, w, 3), dtype=np.uint16)
@@ -366,23 +365,24 @@ def test_emulated_depth_cvtcolor_vs_reference(depth_emu, rng):
         assert np.array_equal(depth_emu(g, 8, 3), ref.cvtColor(g, 8, 3)) and np.array_equal(depth_emu(g.astype(np.float32), 9, 4), ref.cvtColor(g.astype(np.float32), 9, 4))
 
 
-def test_emulated_bayer_edge_aware_and_16bit_vs_reference(rng):
-    from oracle.api import Oracle, available
-    if not available("ref"):
-        pytest.skip("oracle/_ref/libocvref.so not built")
-    ref = Oracle("ref")
+def test_emulated_bayer_edge_aware_and_16bit_vs_reference(ref, rng):
     lib = build_emulation("demosaic.cu", "int emu_demosaic_any(const b200cvMat* s, const b200cvMat* d, int code)",
                           "    return b200cv::demosaic_bilinear(s, d, code, nullptr);")
     lib.emu_demosaic_any.argtypes = [ctypes.POINTER(Mat), ctypes.POINTER(Mat), ctypes.c_int]
+
+    def emu(img, code, dcn):
+        depth = 0 if img.dtype == np.uint8 else 2
+        dst = np.zeros(img.shape + (dcn,), img.dtype)
+        ms, md = mat_of(img), mat_of(dst)
+        ms.type = depth; md.type = depth | ((dcn - 1) << 3)
+        assert lib.emu_demosaic_any(ctypes.byref(ms), ctypes.byref(md), code) == 0
+        return dst
+    ref = with_twin(ref, cvtColor=emu)
     for dtype, depth in ((np.uint8, 0), (np.uint16, 2)):
         for (h, w) in [(3, 3), (4, 5), (17, 33), (18, 34)]:
             img = rng.integers(0, 256 if depth == 0 else 65536, (h, w)).astype(dtype)
             for code, dcn in ((135, 3), (136, 3), (137, 3), (138, 3)) + (((46, 3), (49, 3), (140, 4)) if depth else ()):
-                dst = np.zeros((h, w, dcn), dtype)
-                ms, md = mat_of(img), mat_of(dst)
-                ms.type = depth; md.type = depth | ((dcn - 1) << 3)
-                assert lib.emu_demosaic_any(ctypes.byref(ms), ctypes.byref(md), code) == 0
-                assert np.array_equal(dst, ref.cvtColor(img, code, dcn)), "Bayer %s code %d %dx%d" % (np.dtype(dtype).name, code, w, h)
+                assert np.array_equal(emu(img, code, dcn), ref.cvtColor(img, code, dcn)), "Bayer %s code %d %dx%d" % (np.dtype(dtype).name, code, w, h)
 
 
 # ---- cv::integral (integral.cu): six map-only kernels ----------------------------------------------------------------------------------

@@ -215,6 +215,7 @@ def test_port_vs_reference_two_plane(ref, port, rng):
             assert np.array_equal(a, ref.cvtColorYUV(one, code)), "two-plane == one buffer, code %d" % code
 
 
+@pytest.mark.reference_library
 def test_kat_input_is_the_reference_rng_stream(ref):
     """tests/golden/cvtcolor_kat_input.npy was generated by cv::RNG(0).fill(263x255 8UC3, UNIFORM, 0, 255) -- regenerate and compare"""
     img = np.load(os.path.join(GOLD, "cvtcolor_kat_input.npy"))
@@ -388,6 +389,7 @@ def test_port_vs_reference_lanczos4_resize(ref, port, rng):
                 assert np.array_equal(ref.resize(img, (dw, dh), 4), port.resize(img, (dw, dh), 4)), "LANCZOS4 %s %s -> %s cn=%d" % (img.dtype, (sh, sw), (dh, dw), cn)
 
 
+@pytest.mark.reference_library
 def test_reference_sift_front_end_is_reachable(ref, rng):
     """the oracle for SURVEY 8(f) rank 1: cv::SIFT::detectAndCompute of the unmodified reference (keypoints + 128-float descriptors)"""
     small = rng.random((30, 40)).astype(np.float32)
@@ -539,6 +541,7 @@ def test_port_vs_reference_features(ref, port, rng):
             assert_close(pd[o][i], wd[o][i], atol=1e-3, what="sift dog")
 
 
+@pytest.mark.reference_library
 def test_reference_reproduces_the_depth_cvtcolor_hashes(ref):
     """tests/kat_depth.py: the constants the GPU tests compare against were generated from this very library"""
     from kat_depth import KAT_DEPTH, kat_dcn, kat_hash, kat_input
